@@ -16,7 +16,7 @@ Extra keys of the same JSON line (each leg is outside the headline's timed regio
   federated        configs[4]: one round of the federated-learning example shape (rank 0, N = 1)
   reductions       EncryptedVector.sum / dot (fused kernels) against the launch chains they replace
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 Multi-GPU (torchrun, one rank per GPU): the headline batch shards across ranks (weak scaling: `--batch` is the per-GPU
 batch), no data-path collective; the key limbs are broadcast from rank 0 over NCCL.
@@ -39,6 +39,7 @@ if ROOT not in sys.path:
 KEY_BITS = 2048
 DEFAULT_BATCH = 1 << 20
 ROWS_3072 = 1 << 22
+DUMP_ROWS = 1 << 14
 NOMINAL_MAC_PER_CLK_SM = 32.0     # IMAD.WIDE is a half-rate fmaheavy instruction: 4 SMSPs x 16 lanes / 2
 
 
@@ -454,6 +455,18 @@ def sample_indices(B, count, seed):
     return sorted(idx)
 
 
+def dump_outputs(out_dir, dev, np, B, outputs):
+    """--dump-outputs: the same seeded sample of rows of each [B, limbs] int32 output every run, written as
+    out_dir/<name>.npy in float64 (u32 limbs are exact there), with the sampled row numbers in out_dir/rows.npy.
+    DUMP_ROWS rows of the 2048-bit outputs (128 + 64 limbs) come to 25 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = sample_indices(B, DUMP_ROWS, 2024)
+    ti = dev.torch.tensor(idx, device="cuda")
+    np.save(os.path.join(out_dir, "rows.npy"), np.asarray(idx, dtype=np.float64))
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t[ti].cpu().numpy().view(np.uint32).astype(np.float64))
+
+
 # --------------------------------------------------------------------------------------------- legs
 def leg_headline(dev, args, pb, np, key, pool):
     torch = dev.torch
@@ -511,6 +524,8 @@ def leg_headline(dev, args, pb, np, key, pool):
     dec_ms = sum(dec_each) / args.steps
     enc_ms, dec_ms = dev.max_over_ranks([enc_ms, dec_ms])
     clocks = sampler.stop() if dev.rank == 0 else None
+    if args.dump_outputs and dev.rank == 0:
+        dump_outputs(args.dump_outputs, dev, np, B, {"ciphertexts": d_c, "plaintexts": d_d})
 
     # ---- end to end through the host-pointer C ABI, pinned host buffers, same batch
     e2e = None
@@ -898,7 +913,12 @@ def main():
     ap.add_argument("--reduce-rows", type=int, default=100000)
     ap.add_argument("--fed-dim", type=int, default=100000)
     ap.add_argument("--fed-cpu-sample", type=int, default=60)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of rows of the last step's ciphertexts and decrypted "
+                         "plaintexts to DIR/*.npy (rank 0's shard when --gpus > 1)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 headline leg")
     # the contract is ONE JSON line on stdout: native libraries (NCCL's version banner, ...) write to fd 1 as well, so
     # everything but the final line is sent to stderr
     global _OUT

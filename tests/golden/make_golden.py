@@ -1,12 +1,11 @@
 #!/usr/bin/env python3
 """Generate the golden fixtures in tests/golden/ by running the UNMODIFIED reference.
 
-Run in the build container only (it needs /root/reference, which does not exist on the
-GPU box):
+It needs a checkout of python-paillier 1.5.0, named by PHE_SOURCE_DIR:
 
-    python tests/golden/make_golden.py            # writes tests/golden/*.json
+    PHE_SOURCE_DIR=<checkout> python tests/golden/make_golden.py            # writes tests/golden/*.json
 
-Everything is produced by ``phe`` 1.5.0 imported from /root/reference (pure-Python
+Everything is produced by ``phe`` 1.5.0 imported from that checkout (pure-Python
 bigint branch, phe/util.py:47-48 -- gmpy2 is not installable offline; both branches
 return identical integers, see oracle/paillier_oracle.py).  Keys come from the
 reference's own ``generate_paillier_keypair`` (phe/paillier.py:37-68) and are persisted
@@ -17,7 +16,7 @@ import os
 import random
 import sys
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["PHE_SOURCE_DIR"])
 import phe                                            # noqa: E402
 from phe import paillier, util                        # noqa: E402
 import numpy as np                                    # noqa: E402
@@ -177,6 +176,21 @@ def make_config1(pk, sk):
     return {"n": H(pk.n), "p": H(sk.p), "q": H(sk.q), "rows": rows}
 
 
+def make_is_prime():
+    """The reference's probable-prime test (phe/util.py:421-443) on known primes, Carmichael numbers, strong
+    pseudoprimes to small bases, semiprimes and random odd numbers (all above its small-prime table)."""
+    rng = random.Random(5)
+    primes = [2 ** 127 - 1, 2 ** 521 - 1, (1 << 255) - 19, 2 ** 89 - 1]
+    carmichael = [561, 41041, 825265, 321197185, 5394826801, 232250619601, 9746347772161, 1436697831295441,
+                  60977817398996785, 7156857700403137441, 1791562810662585767521, 87674969936234821377601]
+    strong_pseudo = [3215031751, 3825123056546413051, 318665857834031151167461]   # strong pseudoprimes to bases 2, 3, 5, 7 (and more)
+    semiprimes = [(2 ** 127 - 1) * ((1 << 255) - 19), (2 ** 89 - 1) * (2 ** 107 - 1)]
+    composites = [c for c in carmichael + strong_pseudo + semiprimes if c > 20000]
+    randoms = [rng.getrandbits(256) | 1 | (1 << 255) for _ in range(24)] + [rng.getrandbits(700) | 1 | (1 << 699) for _ in range(6)]
+    return {"known_primes": [H(c) for c in primes], "known_composites": [H(c) for c in composites], "random": [H(c) for c in randoms],
+            "is_prime": [bool(util.is_prime(c)) for c in primes + composites + randoms]}
+
+
 def main():
     # the reference's own known answers (phe/tests/paillier_test.py:128-149, util_test.py:31-44)
     kat = {"n": 126869, "p": 293, "q": 433, "m": 10100, "r": 74384, "c": 935906717,
@@ -188,6 +202,7 @@ def main():
     assert pk.raw_encrypt(10100, 74384) == 935906717 and sk.raw_decrypt(935906717) == 10100
     assert (sk.psquare, sk.qsquare, sk.p_inverse, sk.hp, sk.hq) == (85849, 187489, 300, 203, 133)
     json.dump(kat, open(os.path.join(HERE, "kat_reference_tests.json"), "w"), indent=1)
+    json.dump(make_is_prime(), open(os.path.join(HERE, "is_prime_reference.json"), "w"), indent=0)
 
     for kb, nvec in [(64, 32), (256, 32), (512, 32), (1024, 48), (2048, 32), (3072, 16), (4096, 8)]:
         fx, pk, sk = make_key_fixture(kb, nvec, seed=1000 + kb)

@@ -2,13 +2,10 @@
 generate_paillier_keypairs on the host simulation -- probable-prime agreement with the reference's is_prime
 (phe/util.py:420-443) on primes, composites, Carmichael numbers and strong pseudoprimes to small bases."""
 import importlib
-import os
-import random
-import sys
 
 import pytest
 
-REF = "/root/reference"
+from oracle.golden import H, load_golden
 
 
 @pytest.fixture(scope="module")
@@ -20,36 +17,14 @@ def env(pkg):
     engine_mod._set_engine_for_tests(None)
 
 
-def _ref_is_prime():
-    if not os.path.isdir(os.path.join(REF, "phe")):
-        return None
-    saved = {k: v for k, v in sys.modules.items() if k == "phe" or k.startswith("phe.")}
-    for k in saved:
-        del sys.modules[k]
-    sys.path.insert(0, REF)
-    try:
-        return importlib.import_module("phe.util").is_prime
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "phe" or k.startswith("phe.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-
-
 def test_miller_rabin_batch_agrees_with_the_reference(pkg, env):
+    """Verdicts of the reference's is_prime on the same candidates are stored in tests/golden/is_prime_reference.json."""
     util, engine_mod = env
-    rng = random.Random(5)
-    ref = _ref_is_prime() or util.is_prime
-    primes = [2 ** 127 - 1, 2 ** 521 - 1, (1 << 255) - 19, 2 ** 89 - 1]
-    carmichael = [561 * 1, 41041, 825265, 321197185, 5394826801, 232250619601, 9746347772161, 1436697831295441,
-                  60977817398996785, 7156857700403137441, 1791562810662585767521, 87674969936234821377601]
-    strong_pseudo = [3215031751, 3825123056546413051, 318665857834031151167461]      # strong pseudoprimes to bases 2, 3, 5, 7 (and more)
-    semiprimes = [(2 ** 127 - 1) * ((1 << 255) - 19), (2 ** 89 - 1) * (2 ** 107 - 1)]
-    randoms = [rng.getrandbits(256) | 1 | (1 << 255) for _ in range(24)] + [rng.getrandbits(700) | 1 | (1 << 699) for _ in range(6)]
-    cands = [c for c in primes + carmichael + strong_pseudo + semiprimes + randoms if c > 20000]
-    got = util.is_prime_batch(cands)
-    assert got == [bool(ref(c)) for c in cands]
-    assert got[:4] == [True] * 4 and not any(got[4:4 + len([c for c in carmichael if c > 20000]) + len(strong_pseudo) + len(semiprimes)])
+    fx = load_golden("is_prime_reference.json")
+    primes, composites, randoms = ([H(c) for c in fx[k]] for k in ("known_primes", "known_composites", "random"))
+    got = util.is_prime_batch(primes + composites + randoms)
+    assert got == fx["is_prime"]
+    assert got[:len(primes)] == [True] * len(primes) and not any(got[len(primes):len(primes) + len(composites)])
     # raw kernel on survivors only (no trial division): the pseudoprimes must still fall to random bases
     raw = engine_mod.miller_rabin_batch([3215031751, 2 ** 127 - 1, 3825123056546413051, 318665857834031151167461, 2 ** 61 - 1], rounds=25)
     assert raw == [False, True, False, False, True]

@@ -1,108 +1,103 @@
-"""The boundary exercised the way the reference would bind it: the UNMODIFIED /root/reference/phe package with its three
-bigint seam functions (phe/util.py:38,53,85, imported by name at phe/paillier.py:29) rebound to
-integration/phe_b200_backend.py -- the ctypes stub INTEGRATION.md section 1 quotes -- exactly as the reference's own tests
-flip backends (phe/tests/util_test.py:64-75).  The reference's PaillierTestRawEncryption and PaillierTestEncryptedNumber
-classes (phe/tests/paillier_test.py:106-164, 430-1058) and its util tests then run on the reference's own classes.
-Build container only (needs /root/reference); the engine is the test-only host simulation of the device code."""
-import importlib
+"""The boundary exercised the way the reference would bind it: the three bigint seam functions of the unmodified phe
+package (phe/util.py:38,53,85, imported by name at phe/paillier.py:29) rebound to integration/phe_b200_backend.py --
+the ctypes stub INTEGRATION.md section 1 quotes -- exactly as the reference's own tests flip backends
+(phe/tests/util_test.py:64-75).  tests/golden/make_upstream_traces.py ran the reference's unit tests on the unmodified
+reference and recorded every seam call its phe made (arguments and result, tagged with the test class); here every
+recorded call goes through the backend and must give the same result.  The engine is the test-only host simulation of
+the device code."""
 import importlib.util
 import os
 import sys
-import unittest
+import types
 
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "phe", "tests")), reason="reference tree not present")
+from oracle.golden import load_golden
 
 
 @pytest.fixture(scope="module")
-def real_phe():
+def backend():
     import __graft_entry__ as ge
-    lib = ge.build_hostsim()
-    saved_mods = {k: v for k, v in sys.modules.items() if k == "phe" or k.startswith("phe.")}
-    for k in saved_mods:
-        del sys.modules[k]
-    sys.path.insert(0, REF)
-    try:
-        phe = importlib.import_module("phe")
-        assert os.path.realpath(phe.__file__).startswith(REF), "must be the reference's own package"
-        spec = importlib.util.spec_from_file_location("phe_b200_backend", os.path.join(ge.ROOT, "integration", "phe_b200_backend.py"))
-        backend = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(backend)
-        backend.install(phe, lib_path=lib)
-        yield phe, backend
-        backend.uninstall(phe)
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "phe" or k.startswith("phe.")]:
-            del sys.modules[k]
-        sys.modules.update(saved_mods)
-
-
-def _classes(mod, names):
-    suite = unittest.TestSuite()
-    for n in names:
-        suite.addTests(unittest.defaultTestLoader.loadTestsFromTestCase(getattr(mod, n)))
-    return suite
-
-
-def test_seam_is_rebound_and_counts_calls(real_phe):
-    phe, backend = real_phe
-    import phe.paillier as pp
-    import phe.util as pu
-    assert pp.powmod is backend.powmod and pp.mulmod is backend.mulmod and pp.invert is backend.invert
-    assert pu.powmod is backend.powmod
-    # the reference's known answer (phe/tests/paillier_test.py:128-136) through the reference's own class
-    pk = pp.PaillierPublicKey(126869)
-    sk = pp.PaillierPrivateKey(pk, 293, 433)
-    assert pk.raw_encrypt(10100, 74384) == 935906717 and sk.raw_decrypt(935906717) == 10100
-    # a real-size key: every powmod of encrypt / decrypt goes through the engine (counted by wrapping the backend)
-    calls = {"n": 0}
-    orig = backend._lib.pai_mod_powmod_host
-
-    class Counting:
-        def __call__(self, *a):
-            calls["n"] += 1
-            return orig(*a)
-    backend._lib_saved = backend._lib
-
-    class LibProxy:
-        def __getattr__(self, name):
-            return Counting() if name == "pai_mod_powmod_host" else getattr(backend._lib_saved, name)
-    backend._lib = LibProxy()
-    try:
-        pk2, sk2 = pp.generate_paillier_keypair(n_length=1024)
-        c = pk2.encrypt(-123456.75)
-        assert sk2.decrypt(c + 0.25) == -123456.5
-        assert calls["n"] >= 5          # hp, hq (key constants), r^n, and the CRT pair
-    finally:
-        backend._lib = backend._lib_saved
-
-
-def test_reference_test_classes_on_unmodified_phe(real_phe, monkeypatch):
-    phe, backend = real_phe
-    import phe.paillier as pp
-    orig = pp.generate_paillier_keypair
-    # the simulation is ~100x slower than the GPU: smaller default keys, nothing else changes
-    monkeypatch.setattr(pp, "generate_paillier_keypair",
-                        lambda private_keyring=None, n_length=None: orig(private_keyring, n_length=n_length or 1152))
-    monkeypatch.setattr(phe, "generate_paillier_keypair", pp.generate_paillier_keypair, raising=False)
-    spec = importlib.util.spec_from_file_location("ref_paillier_test_real", os.path.join(REF, "phe", "tests", "paillier_test.py"))
+    spec = importlib.util.spec_from_file_location("phe_b200_backend", os.path.join(ge.ROOT, "integration", "phe_b200_backend.py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
-    assert os.path.realpath(mod.paillier.__file__).startswith(REF)
-    res = unittest.TextTestRunner(verbosity=0).run(_classes(mod, ["PaillierTestRawEncryption", "PaillierTestEncryptedNumber",
-                                                                 "TestKeyring", "TestIssue62"]))
-    assert res.testsRun >= 80
-    assert not res.failures and not res.errors, (res.failures[:2], res.errors[:2])
-    spec = importlib.util.spec_from_file_location("ref_util_test_real", os.path.join(REF, "phe", "tests", "util_test.py"))
-    umod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(umod)
-    res = unittest.TextTestRunner(verbosity=0).run(_classes(umod, ["PaillierUtilTest"]))
-    assert res.testsRun >= 5 and not res.failures and not res.errors, (res.failures[:2], res.errors[:2])
-    spec = importlib.util.spec_from_file_location("ref_math_test_real", os.path.join(REF, "phe", "tests", "math_test.py"))
-    mmod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mmod)
-    res = unittest.TextTestRunner(verbosity=0).run(_classes(mmod, ["ArithmeticTest"]))      # np.mean / np.dot idioms
-    assert res.testsRun >= 2 and not res.failures and not res.errors, (res.failures[:2], res.errors[:2])
+    mod.load(ge.build_hostsim())
+    return mod, load_golden("upstream_seam_trace.json")
+
+
+def _h(s):
+    return -int(s[1:], 16) if s.startswith("-") else int(s, 16)
+
+
+def _replay(fns, calls):
+    bad = []
+    for c in calls:
+        try:
+            got = hex(fns[c["f"]](*[_h(a) for a in c["a"]]))
+        except ZeroDivisionError:
+            got = "ZeroDivisionError"
+        if got != c.get("out", c.get("exc")):
+            bad.append((c["cls"], c["f"], c["a"], got))
+    return bad
+
+
+def test_seam_is_rebound_and_counts_calls(backend):
+    """install() rebinds the seam in phe.util and phe.paillier (a stand-in package with phe's module layout: the
+    backend touches nothing else), uninstall() restores it; the seam calls of the reference's known answer
+    (phe/tests/paillier_test.py:128-136) and of a 1024-bit encrypt / add / decrypt go through the engine."""
+    be, trace = backend
+    names = ("powmod", "mulmod", "invert")
+    pkg, pu, pp = (types.ModuleType(n) for n in ("phe", "phe.util", "phe.paillier"))
+    pkg.util, pkg.paillier = pu, pp
+    originals = {n: (lambda *a: None) for n in names}
+    for mod in (pu, pp):
+        for n in names:
+            setattr(mod, n, originals[n])
+    saved = {k: sys.modules.get(k) for k in ("phe", "phe.util", "phe.paillier")}
+    sys.modules.update({"phe": pkg, "phe.util": pu, "phe.paillier": pp})
+    try:
+        be.install(pkg)
+        assert pp.powmod is be.powmod and pp.mulmod is be.mulmod and pp.invert is be.invert
+        assert pu.powmod is be.powmod and pu.mulmod is be.mulmod and pu.invert is be.invert
+        calls = {"n": 0}
+        lib = be._lib
+
+        class LibProxy:
+            def __getattr__(self, name):
+                fn = getattr(lib, name)
+                if name != "pai_mod_powmod_host":
+                    return fn
+
+                def counted(*a):
+                    calls["n"] += 1
+                    return fn(*a)
+                return counted
+        be._lib = LibProxy()
+        try:
+            fns = {n: getattr(pp, n) for n in names}
+            assert not _replay(fns, trace["flows"]["known_answer"])
+            assert calls["n"] >= 2                    # r^n mod n^2 and the decrypt's powmod
+            calls["n"] = 0
+            assert not _replay(fns, trace["flows"]["roundtrip_1024"])
+            assert calls["n"] >= 5                    # hp, hq (key constants), r^n, and the CRT pair
+        finally:
+            be._lib = lib
+        be.uninstall(pkg)
+        assert all(getattr(mod, n) is originals[n] for mod in (pu, pp) for n in names)
+    finally:
+        for k, v in saved.items():
+            if v is None:
+                sys.modules.pop(k, None)
+            else:
+                sys.modules[k] = v
+
+
+def test_reference_test_classes_on_unmodified_phe(backend):
+    be, trace = backend
+    calls = trace["calls"]
+    classes = {c["cls"] for c in calls}
+    assert {"PaillierTestRawEncryption", "PaillierTestEncryptedNumber", "TestKeyring", "TestIssue62", "PaillierUtilTest",
+            "ArithmeticTest"} <= classes and len(calls) >= 100
+    assert {c["f"] for c in calls} == {"powmod", "mulmod", "invert"}
+    bad = _replay({"powmod": be.powmod, "mulmod": be.mulmod, "invert": be.invert}, calls)
+    assert not bad, (len(bad), bad[:2])

@@ -1,64 +1,24 @@
-"""Run the REFERENCE'S OWN unit tests (phe/tests/paillier_test.py, util_test.py, math_test.py) against the
-drop-in package, with `phe` aliased to python-paillier_b200 and the kernels on the test-only host simulation.
-Only possible where /root/reference exists (the build container); skipped elsewhere.  Key sizes are reduced
-(the simulation is ~100x slower than the GPU), nothing else is changed."""
+"""The REFERENCE'S OWN unit tests (phe/tests/paillier_test.py, util_test.py, math_test.py) replayed on the drop-in
+package, with the kernels on the test-only host simulation.  tests/golden/make_upstream_traces.py ran those tests on
+the unmodified reference and recorded every call their code made into the phe API (keys, arguments, the random r each
+encryption drew, the result or the exception raised); here every recorded call is made again on this package and must
+give the same result, bit for bit, or raise the same exception.  Key sizes are reduced to 1152 bits (the simulation is
+~100x slower than the GPU), nothing else is changed."""
 import importlib
-import os
-import sys
-import unittest
 
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "phe", "tests")), reason="reference tree not present")
+from oracle.golden import load_golden
+from oracle.trace import Loader, dump
 
 
 @pytest.fixture(scope="module")
-def aliased(pkg):
+def trace(pkg):
     import __graft_entry__ as ge
     engine_mod = importlib.import_module("python-paillier_b200.engine")
     engine_mod._set_engine_for_tests(pkg.Engine(ge.build_hostsim()))
-    saved = {k: sys.modules.get(k) for k in ("phe", "phe.paillier", "phe.util", "phe.encoding")}
-    sys.modules["phe"] = pkg
-    sys.modules["phe.paillier"] = importlib.import_module("python-paillier_b200.paillier")
-    sys.modules["phe.util"] = importlib.import_module("python-paillier_b200.util")
-    sys.modules["phe.encoding"] = importlib.import_module("python-paillier_b200.encoding")
-    pkg.paillier = sys.modules["phe.paillier"]
-    pkg.encoding = sys.modules["phe.encoding"]
-    pmod = sys.modules["phe.paillier"]
-    orig = pmod.generate_paillier_keypair
-
-    def small_keys(private_keyring=None, n_length=None):
-        return orig(private_keyring, n_length=n_length or int(os.environ.get("PAI_REFTEST_KEYBITS", "1152")))
-    pmod.generate_paillier_keypair = small_keys
-    pkg.generate_paillier_keypair = small_keys
-    yield pkg
-    pmod.generate_paillier_keypair = orig
-    pkg.generate_paillier_keypair = orig
-    for k, v in saved.items():
-        if v is None:
-            sys.modules.pop(k, None)
-        else:
-            sys.modules[k] = v
+    yield load_golden("upstream_api_trace.json")
     engine_mod._set_engine_for_tests(None)
-
-
-def _load(path, name):
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
-def _run(mod, skip=()):
-    suite = unittest.TestSuite()
-    loader = unittest.TestLoader()
-    for t in loader.loadTestsFromModule(mod):
-        for case in t:
-            if not any(s in case.id() for s in skip):
-                suite.addTest(case)
-    res = unittest.TextTestRunner(verbosity=0).run(suite)
-    return res
 
 
 @pytest.fixture(params=["thread-per-ciphertext", "warp-per-ciphertext"])
@@ -68,18 +28,39 @@ def kernel_family(request, monkeypatch):
     monkeypatch.setenv("PAI_COOP_MAX", "0" if request.param.startswith("thread") else "1000000")
 
 
-def test_reference_paillier_tests(aliased, kernel_family):
-    mod = _load(os.path.join(REF, "phe", "tests", "paillier_test.py"), "ref_paillier_test")
-    # skipped: key-generation sweeps up to 4096 bits / 100 keys (out of the hot-path scope, hours in simulation)
-    res = _run(mod, skip=("testKeyUniqueness", "testDefaultKeySize", "testStaticPrivateKeySize"))
-    assert res.testsRun > 150
-    assert not res.failures and not res.errors, (res.failures[:2], res.errors[:2])
+def _replay(pkg, records, keys):
+    """Re-make every recorded call on this package; returns the calls whose result differs."""
+    util = importlib.import_module("python-paillier_b200.util")
+    ld = Loader(pkg, keys)
+    bad = []
+    for rec in records:
+        args = [ld.load(a) for a in rec["a"]]
+        kw = {k: ld.load(v) for k, v in rec["k"].items()}
+        owner, meth = rec["f"].split(".", 1)
+        fn = getattr(util, meth) if owner == "util" else getattr(args.pop(0), meth)
+        if rec["r"] and meth in ("encrypt", "raw_encrypt") and len(args) < (3 if meth == "encrypt" else 2) \
+                and kw.get("r_value") is None:
+            kw["r_value"] = int(rec["r"][0], 16)      # the r the reference drew (it obfuscates with it)
+        try:
+            got, exc = dump(fn(*args, **kw)), None
+        except Exception as e:                        # noqa: BLE001
+            got, exc = None, type(e).__name__
+        if (exc != rec["exc"]) if "exc" in rec else (exc is not None or got != rec["out"]):
+            bad.append((rec["f"], rec.get("exc", rec.get("out")), exc or got))
+    return bad
 
 
-def test_reference_util_and_math_tests(aliased, kernel_family):
-    mod = _load(os.path.join(REF, "phe", "tests", "util_test.py"), "ref_util_test")
-    res = _run(mod, skip=("Fallbacks",))        # the fallback class toggles phe.util.HAVE_GMP / HAVE_CRYPTO internals
-    assert res.testsRun >= 5 and not res.failures and not res.errors, (res.failures[:2], res.errors[:2])
-    mod = _load(os.path.join(REF, "phe", "tests", "math_test.py"), "ref_math_test")
-    res = _run(mod)
-    assert res.testsRun >= 2 and not res.failures and not res.errors, (res.failures[:2], res.errors[:2])
+def test_reference_paillier_tests(pkg, trace, kernel_family):
+    recs = trace["paillier"]
+    assert trace["tests_run"]["paillier_test"] > 150 and len(recs) > 100
+    assert {r["f"].split(".")[0] for r in recs} >= {"PaillierPublicKey", "PaillierPrivateKey", "EncryptedNumber", "EncodedNumber"}
+    bad = _replay(pkg, recs, trace["keys"])
+    assert not bad, (len(bad), bad[:3])
+
+
+def test_reference_util_and_math_tests(pkg, trace, kernel_family):
+    recs = trace["util_math"]
+    assert trace["tests_run"]["util_test"] >= 5 and trace["tests_run"]["math_test"] >= 2 and len(recs) > 200
+    assert {r["m"] for r in recs} == {"util_test", "math_test"}
+    bad = _replay(pkg, recs, trace["keys"])
+    assert not bad, (len(bad), bad[:3])
